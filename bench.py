@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
            --master-port P bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference --steps 5 --warmup 1      # restated reference CPU path (oracle)
+    python bench.py --steps 20 --warmup 3 --dump-outputs DIR   # also write the last timed step's results as DIR/*.npy
 
 One "step" = STEP_BATCHES (32) passes of the fused hot path (dim_refine: 4 x render -> bbox+zoom -> FlowNetS ->
 se3 compose), each over one batch of 16 synthetic instances = 512 refinements; workload = BASELINE.json configs[1]
@@ -253,6 +254,12 @@ def run_b200(args):
     torch.cuda.synchronize()  # a context must only ever be driven from one stream at a time
     device_pass(prec, W_steps, False)                               # W warm-up steps of the timed configuration
     ms_total, launches, clocks, out = device_pass(prec, K_steps, True)
+    dumped = None
+    if args.dump_outputs:
+        # each stream's persistent result tensors hold its latest batch until the next pass reuses them: the last
+        # len(streams) batches of the last timed step, in batch order (a fixed sample of the step's SB batches)
+        ks = range(max(0, K_steps * SB - len(streams)), K_steps * SB)
+        dumped = {name: np.stack([outs[k % len(streams)][name].cpu().numpy() for k in ks]) for name in out}
     poses_last = out["poses"][-1].cpu().numpy()
     idx_last = (K_steps * SB - 1) % len(sets)
 
@@ -367,7 +374,16 @@ def run_b200(args):
         dist.destroy_process_group()
     refiner.close()
     if result is not None:
+        if dumped is not None:
+            dump_outputs(args.dump_outputs, dumped)
         print(json.dumps(result), flush=True)
+
+
+def dump_outputs(d, arrays):
+    """DIR/<name>.npy, one leading axis over the dumped batches; the int32 bbox indices are widened (exactly) to float64."""
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), a if a.dtype in (np.float32, np.float64) else a.astype(np.float64))
 
 
 def train_on_sets(meshes, sets, B, K, means, device, steps, torch):
@@ -555,7 +571,12 @@ def main():
                     help="c2 = headline config (default); c3 = 13 meshes round-robin; c5 = 50k-vert rasteriser stress mesh")
     ap.add_argument("--workload", default="refine", choices=["refine", "train"],
                     help="refine = the headline metric (default); train = config C4 training step (tools/train_bench.py)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps write the refine results (poses, se3, zoom_factor, bbox) of the last timed step's "
+                         "last --slots batches as DIR/<name>.npy, so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.dump_outputs and (args.workload != "refine" or args.impl != "b200"):
+        ap.error("--dump-outputs applies to the b200 refine workload")
     if args.workload == "train":  # secondary workload: BASELINE.json configs[3]; same launch contract (torchrun for N > 1)
         sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "tools"))
         import train_bench
